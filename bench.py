@@ -66,7 +66,14 @@ def parse():
     p.add_argument("--log-appends", action="store_true",
                    help="experiment (SURVEY 8(f)-1): a second host thread appends entry payloads to the HBM entry buffer "
                         "(rafting_log_append, its own stream) during the whole timed region; the line gains run.log_appends")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR",
+                   help="after the timed steps, write the outbox of the last launch of the last timed step as DIR/<column>.npy "
+                        "(float64, at most 64 MB in all: a fixed sample of groups, listed in gids.npy), so that two builds can be "
+                        "compared output for output")
+    args = p.parse_args()
+    if args.steps < 1:
+        p.error("--steps must be at least 1")
+    return args
 
 
 def b_ack(R):                      # SURVEY.md §8(d): B_ack(R) = 184 + 8 (R - 2)
@@ -294,7 +301,7 @@ def run_cpu_sample(args, threads, steps, warmup, launches, seed):
     total_s, total_acks = float(np.sum(step_s)), int(np.sum(step_acks))
     rates = np.array(step_acks) / np.array(step_s)
     return {"value": total_acks / total_s, "acks": total_acks, "seconds": total_s, "steps": len(step_s),
-            "ms_per_step": 1e3 * total_s / len(step_s), "replay_ok": replay_ok,
+            "ms_per_step": 1e3 * total_s / len(step_s), "replay_ok": replay_ok, "last_outbox": outs[(n_pass - 1) % 2],
             "median_rate": float(np.median(rates)), "min_rate": float(rates.min()), "max_rate": float(rates.max()),
             "sample": f"{G} groups x {rows} ticks x {launches} passes per step x {len(step_s)} steps of the same keyed stream "
                       f"(first {G} group ids, {total_acks} acks, {total_s:.1f} s of CPU wall time), in-memory log, {threads} pinned loop "
@@ -312,6 +319,8 @@ def run_reference(args):
     seed = SEED2 if world == 1 else SEED4
     G = args.groups or (G_CONFIG2 if world == 1 else G_CONFIG4 // world)
     res = run_cpu_sample(args, threads=cores, steps=args.steps, warmup=max(args.warmup, 1), launches=args.cpu_launches, seed=seed)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res["last_outbox"])
     cfg = workload_config(args, world, G)
     line = {
         "impl": "reference", "metric": METRIC, "value": res["value"], "unit": "acks/s",
@@ -490,6 +499,11 @@ def run_engine(args):
     total_ms = ev0.elapsed_time(ev1)
     digest_b = e.digest(0, G)
     replay_ok = bool((digest_a == digest_b).all())
+    if args.dump_outputs:                   # copied now: the passes below reuse the outbox buffers
+        last = abi.Outbox(rows, G, F, G)
+        for name, t in outs[(L - 1) % 2].t.items():
+            getattr(last, name).view(np.uint8).reshape(-1)[:] = t.cpu().numpy()
+        dump_outputs(args.dump_outputs, last, DUMP_BYTES // world, f"rank{rank}_" if world > 1 else "")
 
     # ---- the gathered vector of the timed region's LAST launch against the ranks' own commit columns ----
     gather_ok = None
@@ -819,6 +833,51 @@ def run_engine(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+# ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path hands its caller, so that two builds can be compared output for output
+# ------------------------------------------------------------------------------------------------
+DUMP_BYTES, DUMP_SEED = 60 << 20, 0x5EED00D0       # array bytes; with the .npy headers the files stay under 64 MB
+
+
+def as_float64(a):
+    """A column as float64 without loss: (x, y) pairs and the bit-packed 64-bit meta words (as 32-bit halves, low
+    first) gain a last axis of 2; terms, indices and clocks are converted whole and checked to round-trip."""
+    from rafting_b200 import abi
+    if a.dtype == abi.I64X2:
+        a = np.stack([a["x"], a["y"]], axis=-1)
+    elif a.dtype == np.uint64:
+        a = np.stack([a & np.uint64(0xFFFFFFFF), a >> np.uint64(32)], axis=-1)
+    f = a.astype(np.float64)
+    if not np.array_equal(f.astype(a.dtype), a):
+        raise SystemExit("bench.py --dump-outputs: an output value has no exact float64 form")
+    return f
+
+
+def dump_outputs(out_dir, ob, budget=DUMP_BYTES, prefix=""):
+    """Writes the host outbox `ob` as <out_dir>/<prefix><column>.npy for a sample of groups drawn with a fixed seed (all
+    groups when they fit `budget`); <prefix>gids.npy lists them.  Row columns are [rows, groups(, F)(, 2)], group columns
+    [groups(, 2)].  Payload slots that their meta column marks empty are written as 0: the engine leaves them
+    unwritten, so their bytes are not part of what it computed."""
+    masks = ob.payload_masks()
+
+    def columns(gids):
+        for name, _, _ in ob.ROW_COLS:
+            col = getattr(ob, name)[:, gids]
+            if name in masks:
+                col[~masks[name][:, gids]] = 0
+            yield name, as_float64(col)
+        for name, _ in ob.GROUP_COLS:
+            yield name, as_float64(getattr(ob, name)[gids])
+
+    per_group = 8 + sum(a.nbytes for _, a in columns(np.arange(1)))
+    n = min(ob.n, budget // per_group)
+    gids = np.arange(ob.n) if n == ob.n else np.sort(np.random.default_rng(DUMP_SEED).choice(ob.n, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, prefix + "gids.npy"), gids.astype(np.float64))
+    for name, a in columns(gids):
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), a)
 
 
 _REAL_STDOUT = None

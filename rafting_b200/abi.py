@@ -290,10 +290,17 @@ class Outbox:
     def row_bytes(self) -> bytes:
         return b"".join(getattr(self, name).tobytes() for name, _, _ in self.ROW_COLS)
 
+    def payload_masks(self) -> dict:
+        """Where each payload row column holds a value, as its meta column says: rep_term where a reply exists, plan_*
+        where a plan exists, ballot_* where a ballot exists.  Meta columns are always valid and have no entry."""
+        pm = (self.plan_meta & np.uint64(0xF)) != 0
+        bm = self.ballot_meta != 0
+        return {"rep_term": (self.rep_meta & 1) != 0, "plan_pp": pm, "plan_lc": pm, "plan_epoch": pm,
+                "ballot_term": bm, "ballot_last": bm}
+
     def equal(self, other: "Outbox", gids=None) -> list[str]:
-        """Names of columns that differ.  Payload columns are compared only where their meta column
-        says they are valid (rep_term where a reply exists, plan_* where a plan exists, ballot_* where
-        a ballot exists); group columns only on `gids` if given."""
+        """Names of columns that differ.  Payload columns are compared only where payload_masks() says they
+        are valid; group columns only on `gids` if given."""
         bad = []
 
         def cmp(name, mask=None):
@@ -303,16 +310,9 @@ class Outbox:
             if not np.array_equal(a, b):
                 bad.append(name)
 
-        cmp("rep_meta")
-        cmp("rep_term", (self.rep_meta & 1) != 0)
-        cmp("plan_meta")
-        pm = (self.plan_meta & np.uint64(0xF)) != 0
-        for name in ("plan_pp", "plan_lc", "plan_epoch"):
-            cmp(name, pm)
-        cmp("ballot_meta")
-        bm = self.ballot_meta != 0
-        for name in ("ballot_term", "ballot_last"):
-            cmp(name, bm)
+        masks = self.payload_masks()
+        for name, _, _ in self.ROW_COLS:
+            cmp(name, masks.get(name))
         for name, _ in self.GROUP_COLS:
             cmp(name, gids)
         return bad
